@@ -39,6 +39,7 @@ KIND = os.environ.get("NFB_BENCH_KIND", "ar")  # "ar" (BASELINE config 2) or "co
 FLOPS_PER_SAMPLE_LAYER = {"ar": 1_327_104, "coupled": 933_888}
 MIN_BYTES_PER_SAMPLE_LAYER = 520  # z in + z out + log_q r/w
 METRIC = "samples/sec forward_kld, 32-layer RQ-NSF d=64 batch=65536"
+DUMP_MAX_ROWS = 1 << 22  # --dump-outputs: log_prob rows kept (16 MB of float32)
 
 
 def workload_name(batch=BATCH):
@@ -107,13 +108,13 @@ class ClockSampler(threading.Thread):
 
 # ---------------------------------------------------------------------------------------------------------
 # CPU legs.  `--impl reference` and the GPU line's `cpu_baseline` both time the UNMODIFIED reference package
-# (baseline/_ref/normflows, copied verbatim from /root/reference by __graft_entry__.build()) on the host cores.
+# (oracle/_ref/normflows, installed by __graft_entry__.build(); $NFB_REFERENCE names another checkout) on the host cores.
 # The batch is data-parallel, so it is sharded over worker processes exactly like the GPU arm shards it over
 # GPUs: every worker builds the same model (same seed) with the reference's own classes and runs
 # `model.forward_kld(x_shard)` under no_grad.  The oracle port (oracle/nf_oracle.py) is the fallback only when
-# baseline/_ref is absent (kind "port").
+# no reference is installed (kind "port").
 # ---------------------------------------------------------------------------------------------------------
-REF_DIR = os.path.join(ROOT, "baseline", "_ref")
+REF_DIR = os.environ.get("NFB_REFERENCE") or os.path.join(ROOT, "oracle", "_ref")
 _W = {}
 
 
@@ -137,6 +138,7 @@ def reference_available():
 
 def _use_reference_package():
     """Put the unmodified reference first on sys.path (worker processes / the eager-CUDA leg only)."""
+    assert reference_available(), f"no reference package under {REF_DIR} (run __graft_entry__.build() or set NFB_REFERENCE)"
     assert "normflows" not in sys.modules or sys.modules["normflows"].__file__.startswith(REF_DIR)
     sys.path.insert(0, REF_DIR)
     import normflows as nf
@@ -220,8 +222,8 @@ class CpuReference:
             p.join(timeout=10)
 
     def describe(self, steps, warmup, wall):
-        what = ("unmodified reference package (baseline/_ref/normflows, torch CPU fp32) model.forward_kld under no_grad"
-                if self.use_ref else "oracle/nf_oracle.py (numpy fp32 port; baseline/_ref absent) forward_kld")
+        what = (f"unmodified reference package ({REF_DIR}/normflows, torch CPU fp32) model.forward_kld under no_grad"
+                if self.use_ref else "oracle/nf_oracle.py (numpy fp32 port; no reference installed) forward_kld")
         return (f"{what}; {self.workers} worker processes x {self.threads} torch threads, {self.rows} rows each = "
                 f"{self.rows_total} rows per step, {warmup} warm-up + {steps} timed steps ({wall:.1f} s wall incl. start-up)")
 
@@ -323,7 +325,13 @@ def main():
     ap.add_argument("--no-reference-eager", action="store_true")
     ap.add_argument("--no-train-step", action="store_true")
     ap.add_argument("--no-extra-configs", action="store_true", help="skip BASELINE configs C1 / C2' / C3 / C5 (extra keys)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after timing, write DIR/<name>.npy (rank 0): the losses the timed forward_kld and host-entry "
+                         "passes returned in their last step, and rank 0's per-sample log_prob of the last timed batch "
+                         f"(a seeded sample of {DUMP_MAX_ROWS} rows above that size)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     if args.impl == "reference":
         return run_reference(args)
     if args.impl == "reference-eager":
@@ -351,7 +359,7 @@ def main():
         torch.cuda.synchronize()
         dist.barrier()
     warmup = max(3, args.warmup)
-    steps = max(1, args.steps)
+    steps = args.steps
     B = args.batch
 
     model = build_model().to(dev)
@@ -414,6 +422,20 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         e2e_s = float(t)
     clocks = sampler.stop()
+
+    if args.dump_outputs and rank == 0:
+        # Inputs and weights are seeded, so two builds given the same arguments can be compared output for output.
+        # forward_kld / forward_kld_host are what the timed passes returned (at --gpus N, forward_kld is reduced over
+        # all ranks).  log_prob is recomputed after timing on rank 0's last timed batch -- the per-sample values its
+        # share of that loss averages -- and sampled (fixed seed) to DUMP_MAX_ROWS rows so the files stay under 64 MB.
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        lp = model.log_prob(xs[(steps - 1) % nbuf]).float().cpu().numpy()
+        if lp.size > DUMP_MAX_ROWS:
+            lp = lp[np.sort(np.random.default_rng(0).choice(lp.size, DUMP_MAX_ROWS, replace=False))]
+        outs = {"forward_kld": np.float64(loss_val), "forward_kld_host": np.float64(e2e_loss), "log_prob": lp}
+        for name, a in outs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
 
     # ---- roofline of the dominant kernel (fused spline block), timed live with CUDA events ----
     roof = None
@@ -546,7 +568,7 @@ def main():
             ref = json.loads([ln for ln in out.stdout.splitlines() if ln.startswith("{")][-1])
             line["reference_eager_b200"] = {
                 "value": ref["value"], "unit": "samples/s", "ms_per_step": ref["ms_per_step_median"],
-                "loss": ref["loss"], "how": "baseline/_ref/normflows (unmodified) model.forward_kld under no_grad on "
+                "loss": ref["loss"], "how": f"{REF_DIR}/normflows (unmodified) model.forward_kld under no_grad on "
                 "cuda:0, same model/seed/batch, 10 warm-up + 50 timed passes, CUDA events, median",
                 "speedup_device": value / ref["value"], "speedup_e2e": e2e_value / ref["value"], "target": 10.0}
         except Exception as e:  # reported, never fatal

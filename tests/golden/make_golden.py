@@ -1,7 +1,7 @@
-"""Mint golden vectors from the REAL reference (normflows 1.7.3 at /root/reference).
+"""Mint golden vectors from the REAL reference (normflows 1.7.3).
 
-Run in the build container only (the GPU box has no /root/reference):
-    python tests/golden/make_golden.py
+NFB_REFERENCE names the directory that holds the reference's `normflows` package:
+    NFB_REFERENCE=<normalizing-flows checkout> python tests/golden/make_golden.py
 Writes tests/golden/<case>.npz, each holding:
     spec (json string), sd__<key> (state_dict arrays), x, [y], and for fp64 & fp32:
     log_prob, z, kld, per-layer log_det (ld__<i>) in the density direction, and
@@ -17,7 +17,7 @@ import sys
 import numpy as np
 import torch
 
-sys.path.insert(0, "/root/reference")
+sys.path.insert(0, os.environ["NFB_REFERENCE"])
 import normflows as nf  # noqa: E402  (the reference)
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -655,3 +655,56 @@ def case_spline_circular():
 
 if __name__ == "__main__" and len(sys.argv) > 1 and sys.argv[1] == "spline_circular":
     case_spline_circular()
+
+
+def case_glow_c3():
+    """BASELINE config 3 at its real shape (examples/glow.ipynb cell 2: L=3, K=16, hidden 256, 3x32x32, 10 classes;
+    48 Glow blocks, 8 M parameters), log_prob in fp64.  The weights are too large to store, so most of them are
+    rebuilt from seeds by the consumer (tests/helpers_glow.py build_glow_c3): the constructor runs under
+    torch.manual_seed(0) in fp32, the model is cast to fp64, and every parameter, in model.parameters() order, gets
+    0.02 * randn from a Generator seeded with 2; the inputs are torch.rand / torch.randint from a Generator seeded
+    with 1.  Stored: the entries that recipe does not reproduce (the data-dependent ActNorm statistics), a
+    (sum, sum of squares) checksum of every state_dict entry, a seeded sample of the inputs, and log_prob.
+        python tests/golden/make_golden.py glow_c3"""
+    L, K, hidden, shape, ncls, batch = 3, 16, 256, (3, 32, 32), 10, 64
+    torch.manual_seed(0)
+    q0, merges, flows = [], [], []
+    for i in range(L):
+        flows_ = [nf.flows.GlowBlock(shape[0] * 2 ** (L + 1 - i), hidden, split_mode="channel", scale=True)
+                  for _ in range(K)]
+        flows += [flows_ + [nf.flows.Squeeze()]]
+        if i > 0:
+            merges += [nf.flows.Merge()]
+            ls = (shape[0] * 2 ** (L - i), shape[1] // 2 ** (L - i), shape[2] // 2 ** (L - i))
+        else:
+            ls = (shape[0] * 2 ** (L + 1), shape[1] // 2 ** L, shape[2] // 2 ** L)
+        q0 += [nf.distributions.ClassCondDiagGaussian(ls, ncls)]
+    model = nf.MultiscaleFlow(q0, flows, merges).double()
+    seeded = {k: v.detach().clone() for k, v in model.state_dict().items()}
+    g = torch.Generator().manual_seed(1)
+    x = torch.rand(batch, *shape, generator=g).double()
+    y = torch.randint(ncls, (batch,), generator=g)
+    with torch.no_grad():
+        model.log_prob(x, y)  # ActNorm data-dependent init
+        gp = torch.Generator().manual_seed(2)
+        for k, p in model.named_parameters():  # move the zero-initialised last convolutions / base off their init
+            d = 0.02 * torch.randn(p.shape, generator=gp, dtype=torch.float64)
+            p.add_(d)
+            seeded[k] += d
+        lp = model.log_prob(x, y)
+    sd = {k: v.detach() for k, v in model.state_dict().items()}
+    keys = sorted(sd)
+    idx = np.random.default_rng(0).choice(x.numel(), 512, replace=False)
+    out = {"torch_version": torch.__version__, "log_prob_f64": lp.numpy(), "y": y.numpy(), "x_idx": idx,
+           "x_sample": x.flatten()[idx].numpy(), "ck_keys": np.array(keys),
+           "ck": np.array([[float(sd[k].double().sum()), float((sd[k].double() ** 2).sum())] for k in keys])}
+    for k in keys:
+        if not torch.equal(sd[k], seeded[k]):
+            out["sd__" + k] = sd[k].numpy()
+    np.savez_compressed(os.path.join(HERE, "glow_c3.npz"), **out)
+    print("wrote glow_c3:", sum(k.startswith("sd__") for k in out), "stored entries of", len(keys), "; log_prob",
+          lp[:3].numpy())
+
+
+if __name__ == "__main__" and len(sys.argv) > 1 and sys.argv[1] == "glow_c3":
+    case_glow_c3()

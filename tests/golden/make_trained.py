@@ -1,6 +1,6 @@
-"""Mint TRAINED-weight fixtures with the real reference (normflows 1.7.3 at /root/reference).
+"""Mint TRAINED-weight fixtures with the real reference (normflows 1.7.3).
 
-    python tests/golden/make_trained.py            # build container only (needs /root/reference)
+    NFB_REFERENCE=<normalizing-flows checkout> python tests/golden/make_trained.py
 
 The random-perturbation goldens (make_golden.py) have zero-mean, sign-symmetric weights -- the setting the
 tensor-core accumulate-truncation compensation (csrc/nfb_kernels.h kAccStepGain) was calibrated on.  Trained
@@ -19,7 +19,7 @@ import time
 import numpy as np
 import torch
 
-sys.path.insert(0, "/root/reference")
+sys.path.insert(0, os.environ["NFB_REFERENCE"])
 import normflows as nf  # noqa: E402  (the reference)
 
 HERE = os.path.dirname(os.path.abspath(__file__))

@@ -1,6 +1,7 @@
 """bench.py contract checks that need no GPU: the reference arm (`--impl reference`, the unmodified reference
-package from baseline/_ref on the host cores; the oracle port only if that copy is absent) must print ONE JSON line carrying the same metric / unit / workload as the GPU arm plus the keys the driver
-reads; ranks other than 0 print nothing."""
+package installed in oracle/_ref by build(), on the host cores; the oracle port when none is installed) must print
+ONE JSON line carrying the same metric / unit / workload as the GPU arm plus the keys its readers use; ranks other
+than 0 print nothing; --steps below 1 is refused."""
 import json
 import os
 import subprocess
@@ -35,3 +36,9 @@ def test_reference_arm_json_line():
 
 def test_reference_arm_is_rank0_only():
     assert _run({"RANK": "1", "WORLD_SIZE": "2"}) == []
+
+
+def test_steps_below_one_refused():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True,
+                         text=True, timeout=120)
+    assert out.returncode == 2 and "--steps" in out.stderr

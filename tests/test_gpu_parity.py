@@ -5,11 +5,13 @@ Stated tolerance (BASELINE.json north_star): per-sample `log_prob` rtol <= 1e-4 
 per-layer z atol 2e-4, per-layer log_det atol 2e-3 (fp32 conditioning of single spline elements, see
 tests/test_spline_host.py).  The golden vectors were minted from the real reference
 (tests/golden/make_golden.py); the oracle (oracle/nf_oracle.py) is pinned to them on CPU."""
+import os
+
 import numpy as np
 import pytest
 import torch
 
-from conftest import load_golden
+from conftest import GOLDEN, load_golden
 from helpers import annotate_spec, build_model, rel_err
 from oracle import nf_oracle as O
 
@@ -236,7 +238,7 @@ def test_edge_inputs_through_fused_kernel():
 def test_standalone_spline_kernel_edges():
     import ctypes as C
     from normflows import _lib as L
-    f = np.load("tests/golden/spline_edges.npz")
+    f = np.load(os.path.join(GOLDEN, "spline_edges.npz"))
     x = cuda(f["x_f32"].reshape(-1, 1))
     params = cuda(np.concatenate([f["uw_f32"], f["uh_f32"], f["ud_f32"]], axis=1))
     for inv in (0, 1):
@@ -263,7 +265,7 @@ def test_host_entry_points_and_repack():
 
 
 def test_actnorm_data_dependent_init():
-    f = np.load("tests/golden/actnorm_init.npz")
+    f = np.load(os.path.join(GOLDEN, "actnorm_init.npz"))
     an = nf.flows.ActNorm(6).cuda()
     x = f["x"][:, :, 0, 0]  # [8, 6] slice as a 2-D batch
     z, ld = an.inverse(cuda(x))
@@ -367,7 +369,7 @@ def test_conv2d_tensor_core_matches_oracle(shape):
 
 
 def test_glow_actnorm_data_dependent_init_on_images():
-    f = np.load("tests/golden/actnorm_init.npz")
+    f = np.load(os.path.join(GOLDEN, "actnorm_init.npz"))
     blk = nf.flows.GlowBlock(6, 8).cuda()
     z, ld = blk.inverse(cuda(f["x"]))  # first call initialises ActNorm from the batch (normalization.py:33-38)
     an = blk.flows[2]
@@ -381,7 +383,7 @@ def test_backward_matches_reference_gradients(kind):
     """loss.backward() (examples/neural_spline_flow.ipynb cell 4): forward value from the CUDA kernels,
     gradients from the interim autograd hook (normflows/_autograd.py) vs gradients minted from the reference."""
     spec, sd, _ = load_golden(f"nsf_{kind}_d5_h128_l3")
-    g = np.load(f"tests/golden/grads_nsf_{kind}_d5_h128_l3.npz")
+    g = np.load(os.path.join(GOLDEN, f"grads_nsf_{kind}_d5_h128_l3.npz"))
     model = build_model(spec, sd).cuda()
     torch.set_grad_enabled(True)  # (the autouse fixture restores the previous mode)
     for p in model.parameters():
@@ -462,7 +464,7 @@ def test_trained_weights_parity(kind):
     structured 64-d target) -- off the calibration set of the accumulate-truncation compensation (kAccStepGain):
     post-ReLU activations against correlated weights.  log_prob rtol 1e-4 on every row vs the reference's fp64."""
     import json
-    f = np.load(f"tests/golden/trained_{kind}_d64_h256_l4.npz")
+    f = np.load(os.path.join(GOLDEN, f"trained_{kind}_d64_h256_l4.npz"))
     meta = json.loads(str(f["meta"]))
     torch.manual_seed(meta["seed"])  # masks / permutations are functions of the constructor seed
     fl = []
@@ -497,7 +499,7 @@ def test_autoregressive_sampling_fused_d64():
     reference vectors minted by tests/golden/make_golden.py ar64fwd.  The reference's own fp32 run differs from its
     fp64 run by 2.8e-4 on these latents (64 chained spline inversions per layer); bound ours by the same spread."""
     spec, sd, _ = load_golden("nsf_ar_d64_h256_l2")
-    f = np.load("tests/golden/nsf_ar_d64_h256_l2_fwd.npz")
+    f = np.load(os.path.join(GOLDEN, "nsf_ar_d64_h256_l2_fwd.npz"))
     model = build_model(spec, sd).cuda()
     z = cuda(f["z_f64"])
     y0, ld0 = model.flows[0].forward(z)   # one autoregressive layer alone
@@ -653,7 +655,7 @@ def test_backward_flagship_shape_matches_reference(kind, native):
     the interim torch re-materialisation (kept as the A/B reference).  Both against fp64 autograd of the reference."""
     from normflows._autograd import DensityFn
     spec, sd, _ = load_golden(f"nsf_{kind}_d64_h256_l2")
-    g = np.load(f"tests/golden/grads_nsf_{kind}_d64_h256_l2.npz")
+    g = np.load(os.path.join(GOLDEN, f"grads_nsf_{kind}_d64_h256_l2.npz"))
     model = build_model(spec, sd).cuda()
     torch.set_grad_enabled(True)
     DensityFn.use_native_backward = native
@@ -747,7 +749,7 @@ def test_reference_options_glow_logit_temperature_and_callable_nets():
     """Options of in-scope classes that used to raise (VERDICT r1 missing #7), against vectors minted from the reference
     (tests/golden/make_golden.py options): Invertible1x1Conv(use_lu=False), ConvNet2d(actnorm=True),
     MultiscaleFlow(transform=Logit), temperature-annealed base distributions, nets.* called as modules."""
-    f = np.load("tests/golden/options.npz")
+    f = np.load(os.path.join(GOLDEN, "options.npz"))
     model = _build_glow_options(f).cuda()
     x, y = cuda(f["x"]), torch.from_numpy(f["y"]).cuda()
     lp = model.log_prob(x, y).cpu().numpy()
@@ -788,7 +790,7 @@ def test_reference_options_glow_logit_temperature_and_callable_nets():
 def test_neighbour_layers_maf_and_invertible_affine():
     """SURVEY 8f-4: MaskedAffineAutoregressive (one MADE pass forward, D passes inverse) and InvertibleAffine (both
     parameterisations), against vectors minted from the reference (tests/golden/make_golden.py neighbours)."""
-    f = np.load("tests/golden/neighbours.npz")
+    f = np.load(os.path.join(GOLDEN, "neighbours.npz"))
     maf = nf.flows.MaskedAffineAutoregressive(6, 32, num_blocks=2)
     maf.load_state_dict({k[5:]: torch.from_numpy(np.asarray(f[k])) for k in f.files if k.startswith("maf__")}, strict=True)
     maf = maf.cuda()
@@ -828,7 +830,7 @@ def test_residual_flow_matches_reference(d):
     and the power-series estimators with the random truncation and the Hutchinson probe injected (the same values the
     reference was given while tests/golden/make_golden.py residual minted the vectors): eval = basic estimator with 20
     exact terms (:183-192,355-366), training = Neumann surrogate (:368-379)."""
-    f = np.load("tests/golden/residual.npz")
+    f = np.load(os.path.join(GOLDEN, "residual.npz"))
     model = _residual_model(f, d)
     x = cuda(f[f"x{d}"])
     n_inj, eps = f[f"n_inj{d}"], f[f"eps{d}"]
@@ -879,7 +881,7 @@ def test_residual_flow_matches_reference(d):
 def test_conditional_normalizing_flow_with_context():
     """SURVEY 8f-4: ConditionalNormalizingFlow with context-conditioned coupled / autoregressive spline layers (GLU
     context branch) and a ConditionalDiagGaussian base, against the reference (make_golden.py conditional)."""
-    f = np.load("tests/golden/conditional.npz")
+    f = np.load(os.path.join(GOLDEN, "conditional.npz"))
     torch.manual_seed(51)
     d, c = 6, 3
     flows = []
@@ -944,42 +946,18 @@ def test_glow_conditioner_at_real_width(cfg):
     assert np.abs(y - ref).max() <= 1e-4 * scale + 1e-5, (np.abs(y - ref).max(), scale)
 
 
-def test_glow_c3_shape_against_reference_on_this_gpu(tmp_path):
+def test_glow_c3_shape_against_reference_on_this_gpu():
     """BASELINE config 3 at its REAL shape (examples/glow.ipynb cell 2: L=3, K=16, hidden 256, 3x32x32; 48 Glow blocks,
-    8 M parameters -- too large for a committed golden): the unmodified reference (baseline/_ref) is run in fp64 in a
-    separate process on this GPU by tests/ref_runner.py; its state_dict is loaded verbatim and log_prob compared at the
-    stated tolerance (rtol 1e-4 on every row; |log_prob| ~ 1e3-1e4 here)."""
-    import subprocess
-    import sys
-    from conftest import ROOT
-    import os
-    out = str(tmp_path / "glow_c3.npz")
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "ref_runner.py"), "glow_c3", out, "64"],
-                       capture_output=True, text=True, timeout=900)
-    if r.returncode == 3:
-        pytest.skip("baseline/_ref not present (run __graft_entry__.build() where /root/reference exists)")
-    assert r.returncode == 0, r.stderr[-2000:]
-    f = np.load(out)
-    L_, K, hidden, shape, ncls = 3, 16, 256, (3, 32, 32), 10
-    q0, merges, flows = [], [], []
-    for i in range(L_):
-        fl = [nf.flows.GlowBlock(shape[0] * 2 ** (L_ + 1 - i), hidden, split_mode="channel", scale=True)
-              for _ in range(K)] + [nf.flows.Squeeze()]
-        flows += [fl]
-        if i > 0:
-            merges += [nf.flows.ImageMerge()]
-            ls = (shape[0] * 2 ** (L_ - i), shape[1] // 2 ** (L_ - i), shape[2] // 2 ** (L_ - i))
-        else:
-            ls = (shape[0] * 2 ** (L_ + 1), shape[1] // 2 ** L_, shape[2] // 2 ** L_)
-        q0 += [nf.distributions.ClassCondDiagGaussian(ls, ncls)]
-    model = nf.MultiscaleFlow(q0, flows, merges)
-    sd = {k[4:]: torch.from_numpy(np.asarray(f[k])).float() if f[k].dtype.kind == "f" else torch.from_numpy(np.asarray(f[k]))
-          for k in f.files if k.startswith("sd__")}
-    model.load_state_dict(sd, strict=True)
+    8 M parameters): the reference's fp64 log_prob (tests/golden/glow_c3.npz, make_golden.py glow_c3) for weights
+    rebuilt from seeds plus the stored ActNorm statistics, compared at the stated tolerance (rtol 1e-4 on every row;
+    |log_prob| ~ 1e3-1e4 here)."""
+    from helpers_glow import build_glow_c3
+    f = np.load(os.path.join(GOLDEN, "glow_c3.npz"))
+    model, x, y = build_glow_c3(f)
     model = model.cuda()
-    lp = model.log_prob(cuda(f["x"]), torch.from_numpy(f["y"]).cuda()).cpu().numpy().astype(np.float64)
+    lp = model.log_prob(x.cuda(), y.cuda()).cpu().numpy().astype(np.float64)
     rel = np.abs(lp - f["log_prob_f64"]) / np.abs(f["log_prob_f64"])
-    print(f"\\n[glow C3 shape, 64 images] |log_prob| ~ {np.abs(f['log_prob_f64']).mean():.0f}; rel err max {rel.max():.2e} median {np.median(rel):.2e}")
+    print(f"\n[glow C3 shape, 64 images] |log_prob| ~ {np.abs(f['log_prob_f64']).mean():.0f}; rel err max {rel.max():.2e} median {np.median(rel):.2e}")
     assert rel.max() < RTOL, rel.max()
 
 
@@ -989,7 +967,7 @@ def test_circular_spline_layers_match_reference(tag):
     """SURVEY 8f-4: CircularCoupled / CircularAutoregressive RQ splines (per-feature tails list, periodic features in
     front of the conditioner, scalar and per-feature tail bounds) in both directions against vectors minted from the
     reference (tests/golden/make_golden.py circular); reference checkpoints load strict=True."""
-    f = np.load("tests/golden/circular.npz")
+    f = np.load(os.path.join(GOLDEN, "circular.npz"))
     d, tbt = 6, torch.from_numpy(np.asarray(f["tail_bound_tensor"]))
     make = {
         "cc_s": lambda: nf.flows.CircularCoupledRationalQuadraticSpline(d, 2, 32, [0, 2, 5], tail_bound=3.0),
@@ -1025,7 +1003,7 @@ def test_circular_spline_layers_match_reference(tag):
 def test_glow_base_distribution(tag):
     """GlowBase (distributions/base.py:347-471): log_prob against reference-minted vectors (with / without class
     conditioning and temperature); sample() returns (z, log_p) with log_p == log_prob(z)."""
-    f = np.load("tests/golden/glow_base.npz")
+    f = np.load(os.path.join(GOLDEN, "glow_base.npz"))
     q = nf.distributions.GlowBase((4, 3, 3), num_classes=5 if tag == "cc" else None)
     q.load_state_dict({k[len(tag) + 2:]: torch.from_numpy(np.asarray(f[k])) for k in f.files if k.startswith(tag + "__")},
                       strict=True)
@@ -1061,3 +1039,30 @@ def test_host_batch_in_flight_repeated_calls():
         for _ in range(2):
             assert model.forward_kld_host(xh) == pytest.approx(ref_kld, rel=1e-6)
             np.testing.assert_array_equal(model.log_prob_host(xh).numpy(), ref_lp)
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs(tmp_path):
+    """bench.py --dump-outputs: the last timed step's loss, the last host-entry step's loss and the per-sample log_prob
+    of the last timed batch, the same on a second run with the same arguments (seeded inputs and weights)."""
+    import json
+    import subprocess
+    import sys
+    from conftest import ROOT
+    runs = []
+    for r in range(2):
+        d = tmp_path / f"run{r}"
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "3", "--warmup", "3",
+                              "--batch", "8192", "--no-cpu-baseline", "--no-reference-eager", "--no-train-step",
+                              "--no-extra-configs", "--dump-outputs", str(d)], capture_output=True, text=True,
+                             timeout=900)
+        assert out.returncode == 0, out.stderr[-2000:]
+        line = json.loads([ln for ln in out.stdout.splitlines() if ln.startswith("{")][-1])
+        assert line["steps"] == 3
+        runs.append({n: np.load(d / f"{n}.npy") for n in ("forward_kld", "forward_kld_host", "log_prob")})
+    a, b = runs
+    assert a["log_prob"].shape == (8192,) and a["log_prob"].dtype == np.float32 and np.isfinite(a["log_prob"]).all()
+    assert float(a["forward_kld"]) == pytest.approx(-float(a["log_prob"].astype(np.float64).mean()), rel=1e-6)
+    assert float(b["forward_kld"]) == line["config"]["loss"]
+    for n in a:
+        np.testing.assert_allclose(a[n], b[n], rtol=1e-6)

@@ -2,10 +2,12 @@
 tests/golden/ was produced by tests/golden/make_golden.py importing normflows 1.7.3.
 fp64 must agree to round-off (the restatement is the same arithmetic); fp32 to a few ulp-ish
 multiples because numpy/OpenBLAS and ATen/MKL order their sums differently."""
+import os
+
 import numpy as np
 import pytest
 
-from conftest import load_golden
+from conftest import GOLDEN, load_golden
 from oracle import nf_oracle as O
 
 NF_CASES = ["nsf_ar_d64_h256_l2", "nsf_ar_d5_h128_l3", "nsf_ar_d2_h32_l2_k4",
@@ -14,7 +16,7 @@ NF_CASES = ["nsf_ar_d64_h256_l2", "nsf_ar_d5_h128_l3", "nsf_ar_d2_h32_l2_k4",
 
 
 def test_spline_edges():
-    f = np.load("tests/golden/spline_edges.npz")
+    f = np.load(os.path.join(GOLDEN, "spline_edges.npz"))
     # fp32: the knot-hit inputs (x[8:15]) sit within one ulp of a bin edge of a possibly very narrow
     # bin (min width 1e-3*2B), so theta moves by ~ulp(x)/width and lad by up to ~1e-4: loose atol there.
     for tag, rtol, atol in (("f64", 1e-12, 1e-13), ("f32", 1e-4, 5e-4)):
@@ -96,7 +98,7 @@ def test_glow_multiscale_both_directions():
 
 
 def test_actnorm_init():
-    f = np.load("tests/golden/actnorm_init.npz")
+    f = np.load(os.path.join(GOLDEN, "actnorm_init.npz"))
     s, t = O.actnorm_init(f["x"], f["s"].shape, "inverse")
     np.testing.assert_allclose(s, f["s"], rtol=1e-12)
     np.testing.assert_allclose(t, f["t"], rtol=1e-12, atol=1e-14)
@@ -117,7 +119,7 @@ def test_gradient_oracle_matches_reference_autograd(kind):
     gradients minted from the reference's own autograd in fp64 (make_golden.py grads): every parameter + input."""
     from oracle import nf_oracle_grad as G
     spec, sd, _ = load_golden(f"nsf_{kind}_d5_h128_l3")
-    g = np.load(f"tests/golden/grads_nsf_{kind}_d5_h128_l3.npz")
+    g = np.load(os.path.join(GOLDEN, f"grads_nsf_{kind}_d5_h128_l3.npz"))
     loss, grads, gx = G.forward_kld_grads(spec, sd, g["x"].astype(np.float64))
     assert loss == pytest.approx(float(g["kld"]), rel=1e-6)  # the reference accumulates log_q in fp32 (core.py:96)
     np.testing.assert_allclose(gx, g["grad__x"], rtol=1e-9, atol=1e-12)
@@ -137,7 +139,7 @@ _CIRC = {"cc_s": ("CircularCoupledRationalQuadraticSpline", [0, 2, 5], False),
 def test_circular_spline_layers_fp64(tag):
     """Circular NSF layers (per-feature tails, periodic features, scalar / per-feature bounds) against vectors minted
     from the reference (tests/golden/make_golden.py circular): both directions, fp64, 1e-10."""
-    f = np.load("tests/golden/circular.npz")
+    f = np.load(os.path.join(GOLDEN, "circular.npz"))
     kind, ind_circ, tensor_tb = _CIRC[tag]
     sd = {"flows.0." + k[len(tag) + 2:]: np.asarray(f[k]) for k in f.files if k.startswith(tag + "__")}
     L = {"type": kind, "features": 6, "ind_circ": ind_circ, "num_bins": 8,
@@ -156,7 +158,7 @@ def test_circular_spline_layers_fp64(tag):
 @pytest.mark.parametrize("tag", ["plain", "cc"])
 def test_glow_base_log_prob_fp64(tag):
     """GlowBase.log_prob (distributions/base.py:436-471) against reference-minted vectors, with and without temperature."""
-    f = np.load("tests/golden/glow_base.npz")
+    f = np.load(os.path.join(GOLDEN, "glow_base.npz"))
     sd = {k[len(tag) + 2:]: np.asarray(f[k]).astype(np.float64) for k in f.files if k.startswith(tag + "__")}
     z = np.asarray(f[f"{tag}_z"], dtype=np.float64)
     y = np.asarray(f[f"{tag}_y"]) if tag == "cc" else None
